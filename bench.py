@@ -54,7 +54,14 @@ def parse():
                     help="engine A/B option (Engine.set_option), e.g. --opt pdl=1 with SGMSE_B200_PDL=1; recorded in config")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the enhanced waveforms of the last timed step (float32 [batch, samples]) "
+                         "to DIR/enhanced.npy (DIR/enhanced_rank<r>.npy per rank when --gpus > 1); inputs, weights and noise "
+                         "seeds are fixed, so two builds run with the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 arm computed")
+    return args
 
 
 def peaks():
@@ -336,6 +343,11 @@ def run_b200(args):
         clocks.start()
     ms = timed(step_dev, args.steps)
     launches = eng.counter("kernel_launches") - l0
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "enhanced.npy" if world == 1 else f"enhanced_rank{rank}.npy"),
+                out_dev.float().cpu().numpy())
     step_host(0)
     ms_e2e = timed(step_host, args.steps)
     clk = clocks.stop() if rank == 0 else None

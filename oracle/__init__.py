@@ -16,8 +16,10 @@ follows.  It is pinned against the live reference (imported from
   configs of all three backbones (forward, score, PC / SB / ODE samplers, the
   enhancement chain, FIR / STFT ops) and ``full_n30.npz``, the reference's own
   full-size N = 30 enhancement of one 4-s clip (BASELINE.json configs[0]), and
-* ``tests/test_oracle_vs_reference.py`` – live comparison at full size, skipped
-  where ``/root/reference`` does not exist (the GPU box).
+* ``tests/test_oracle_vs_reference.py`` – comparison at full size against
+  ``tests/golden/reference_live.npz`` (reference outputs and ScoreModel attribute
+  skeletons, also from ``oracle/make_golden.py``); only its
+  tests that need the reference's ScoreModel class itself run live.
 
 ``oracle/ode.py`` additionally restates a third-party algorithm the reference
 calls (scipy's RK45); it is pinned to the installed scipy itself.

@@ -6,7 +6,9 @@ Every array below is an output of the reference's own modules imported from
 /root/reference (see oracle/refshim.py); the weights are the reference's own
 random init (``torch.manual_seed``), stored so the fixtures travel to the GPU box.
 Configs are reduced (nf=16, 3 levels, F=64) so that the fixtures stay small; the
-full-size comparison against the live reference is tests/test_oracle_vs_reference.py.
+full-size reference outputs of tests/test_oracle_vs_reference.py are reference_live.npz.
+
+    python -m oracle.make_golden reference_live    # reference_live.npz only
 TEST INFRASTRUCTURE – see oracle/__init__.py.
 """
 from __future__ import annotations
@@ -292,6 +294,131 @@ def golden_mid_tc(name="ncsnpp_mid"):
     print(name, "params", sum(v.numel() for v in model.dnn.state_dict().values()))
 
 
+def score_model_skeleton(model) -> dict:
+    """Everything ``sgmse_b200.config_from_score_model`` / ``install`` read from a live ScoreModel, as plain data: the
+    NCSN++ attributes, the type name (and ``out_ch``) of every entry of ``dnn.all_modules``, the data module's STFT
+    settings and window, the SDE and the state_dict layout.  tests/test_oracle_vs_reference.py rebuilds a stand-in from it."""
+    dnn, dm, sde = model.dnn, model.data_module, model.sde
+    d = {"backbone": model.backbone, "t_eps": float(model.t_eps), "sr": int(getattr(model, "sr", 16000)),
+         "dnn": {a: getattr(dnn, a) for a in ("nf", "num_resolutions", "num_res_blocks", "progressive", "progressive_input",
+                                             "resblock_type", "embedding_type", "skip_rescale", "conditional", "centered",
+                                             "scale_by_sigma") if hasattr(dnn, a)},
+         "all_modules": [[type(m).__name__, getattr(m, "out_ch", None)] for m in dnn.all_modules],
+         "data_module": {"transform_type": dm.transform_type, "n_fft": dm.n_fft, "hop_length": dm.hop_length,
+                         "spec_factor": float(dm.spec_factor), "spec_abs_exponent": float(dm.spec_abs_exponent),
+                         "window": dm.window.float().tolist()},
+         "sde": {"type": type(sde).__name__, "N": sde.N,
+                 **{a: float(getattr(sde, a)) for a in ("theta", "sigma_min", "sigma_max", "k", "c", "eps") if hasattr(sde, a)},
+                 **({"sampler_type": sde.sampler_type} if hasattr(sde, "sampler_type") else {})},
+         "state_dict": [[k, list(v.shape)] for k, v in dnn.state_dict().items()]}
+    d["dnn"]["attn_resolutions"] = list(dnn.attn_resolutions)
+    d["dnn"]["all_resolutions"] = list(dnn.all_resolutions)
+    for a in ("loss_type", "network_scaling", "c_in", "c_out", "c_skip", "sigma_data"):
+        if hasattr(model, a):
+            d[a] = getattr(model, a)
+    return d
+
+
+REF_48K = dict(n_fft=1534, hop_length=384, spec_factor=0.065, spec_abs_exponent=0.667, theta=2.0, sigma_min=0.1, sigma_max=1.0)
+REF_V2_SBVE = dict(sde="sbve", k=2.6, c=0.4, sampler_type="sde", N=50, loss_type="data_prediction", network_scaling="1/sigma",
+                   c_in="edm", c_out="edm", c_skip="edm")
+# (theta, sigma_min, sigma_max), N, snr: BASELINE configs 2, 4 and 3
+SCHEDULES = [((1.5, 0.05, 0.5), 30, 0.5), ((1.5, 0.05, 0.5), 50, 0.33), ((2.0, 0.1, 1.0), 30, 0.5)]
+DROPIN_MID = dict(nf=64, ch_mult=(1, 2, 2), image_size=64, attn_resolutions=(16,), num_res_blocks=1, n_fft=126, hop_length=32)
+DROPIN_LENGTHS = [4000, 1900, 3100, 2000]
+
+
+def golden_reference_live(name="reference_live"):
+    """What tests/test_oracle_vs_reference.py and the batched-service test of tests/test_gpu_dropin.py compare with: outputs
+    of the unmodified reference at full size (NCSN++ forward, the enhancement.py:75-96 chain at N = 1), its SDE scalars and
+    sampler schedules, its probability-flow ODE sampler on a 48 kHz configuration, its per-file enhancement loop on a
+    tcgen05-tileable configuration, and the attribute skeletons of three live ScoreModels (JSON, key 'score_models').  Weights are
+    the oracle's seeded init (oracle/weights.py) loaded into the reference model; inputs and noise come from seeds."""
+    import json
+    from . import weights as o_w
+    refshim.import_reference()
+    from sgmse.util.other import pad_spec
+    from sgmse.sdes import OUVESDE
+    from sgmse_b200 import Engine, EngineConfig
+    out, skel = {}, {}
+    cfg = NetConfig.ncsnpp()
+    m16 = refshim.make_score_model("ncsnpp", seed=0)
+    skel["ncsnpp"] = score_model_skeleton(m16)
+    out["fwd_keys"] = np.array(list(m16.dnn.state_dict().keys()))
+    m16.dnn.load_state_dict(o_w.make_state_dict(cfg, seed=0))
+    g = torch.Generator().manual_seed(0)
+    x = torch.complex(torch.randn(1, 2, 256, 64, generator=g), torch.randn(1, 2, 256, 64, generator=g)) * 0.3
+    with torch.no_grad():
+        out["fwd_out"] = _np(m16.dnn(x, torch.tensor([0.4])))
+    ts = torch.tensor([1.0, 0.5, 0.03])
+    out["sde_t"] = _np(ts)
+    out["sde_std"] = np.array([float(m16.sde._std(t[None])) for t in ts])
+    out["sde_diffusion"] = np.array([float(m16.sde.sde(torch.zeros(1), torch.zeros(1), t[None])[1]) for t in ts])
+    # enhancement.py:75-96, N = 1, full-size network, one 0.5-s clip (63 frames -> padded to 64)
+    g = torch.Generator().manual_seed(4)
+    L = 8000
+    wav = 0.1 * torch.randn(1, L, generator=g)
+    draws = sde_mod.make_noise((1, 1, 256, 64), 3, seed=5)
+    norm = wav.abs().max()
+    Y = pad_spec(torch.unsqueeze(m16._forward_transform(m16._stft(wav / norm)), 0))
+    with refshim.injected_noise(draws):
+        smp, nfe = m16.get_pc_sampler("reverse_diffusion", "ald", Y, N=1, corrector_steps=1, snr=0.5)()
+    out["chain_enh"] = _np(m16.to_audio(smp.squeeze(), L) * norm)
+    out["chain_nfe"] = np.int64(nfe)
+    # get_ode_sampler's default denoise=True fails inside the reference (predictors.py:60)
+    try:
+        m16.get_ode_sampler(torch.zeros(1, 1, 256, 64, dtype=torch.complex64), device="cpu", rtol=1e-1, atol=1e-1)()
+        out["ode_default_error"] = np.array("")
+    except TypeError as exc:
+        out["ode_default_error"] = np.array(str(exc))
+    # sampler schedules: the reference's scalars on the engine's own fp32 time steps
+    for i, ((theta, smin, smax), N, snr) in enumerate(SCHEDULES):
+        sde = OUVESDE(theta=theta, sigma_min=smin, sigma_max=smax, N=N)
+        eng = Engine(EngineConfig(theta=theta, sigma_min=smin, sigma_max=smax, t_eps=0.03))
+        ets = eng.sampler_schedule(N=N, predictor="reverse_diffusion", corrector="ald", corrector_steps=1, snr=snr)[0]
+        eng.close()
+        x0 = torch.zeros(1, 1, 1, 1, dtype=torch.complex64)
+        y0 = torch.ones(1, 1, 1, 1, dtype=torch.complex64)
+        std, f, G = [], [], []
+        for j in range(N):
+            t = ets[j:j + 1]
+            stepsize = ets[j] - ets[j + 1] if j != N - 1 else ets[-1]
+            std.append(float(sde._std(t)))
+            fj, Gj = sde.discretize(x0, y0, t, stepsize)
+            f.append(float(fj.real))
+            G.append(float(Gj))
+        out[f"sched{i}_linspace"] = _np(torch.linspace(sde.T, 0.03, N))
+        out[f"sched{i}_ts"] = _np(ets)
+        out[f"sched{i}_std1"] = np.float64(float(sde._std(torch.ones(1))))
+        out[f"sched{i}_std"], out[f"sched{i}_f"], out[f"sched{i}_G"] = np.array(std), np.array(f), np.array(G)
+    # probability-flow ODE, 48 kHz SDE parameters, eps = 0.05, batch of 2 = one coupled ODE system
+    small = dict(nf=16, ch_mult=(1, 2, 2), image_size=64, num_res_blocks=2)
+    m = refshim.make_score_model("ncsnpp_48k", seed=5, n_fft=126, hop_length=32, theta=2.0, sigma_min=0.1, sigma_max=1.0, **small)
+    m.dnn.load_state_dict(o_w.make_state_dict(NetConfig.ncsnpp_48k(**small), seed=5))
+    g = torch.Generator().manual_seed(3)
+    y = torch.complex(torch.randn(2, 1, 64, 64, generator=g), torch.randn(2, 1, 64, 64, generator=g)) * 0.3
+    with refshim.injected_noise(sde_mod.make_noise(tuple(y.shape), 1, seed=23)):
+        smp, nfe = m.get_ode_sampler(y, denoise=False, device="cpu", rtol=1e-3, atol=1e-3, eps=0.05)()
+    out["ode_x"], out["ode_nfe"] = _np(smp), np.int64(nfe)
+    # the reference's per-file loop (enhancement.py:58-99) over clips of four lengths, N = 3
+    mcfg = {k: v for k, v in DROPIN_MID.items() if k not in ("n_fft", "hop_length")}
+    m = refshim.make_score_model("ncsnpp", seed=7, **DROPIN_MID)
+    m.dnn.load_state_dict(o_w.make_state_dict(NetConfig.ncsnpp(**mcfg), seed=7))
+    g = torch.Generator().manual_seed(8)
+    nd = sde_mod.n_noise_draws(3, "reverse_diffusion", "ald", 1)
+    for i, n in enumerate(DROPIN_LENGTHS):
+        clip = (0.1 * torch.randn(n, generator=g) * (1.0 + 0.5 * i))[None]
+        norm = clip.abs().max()
+        Y = pad_spec(torch.unsqueeze(m._forward_transform(m._stft(clip / norm)), 0), mode="zero_pad")
+        with refshim.injected_noise(sde_mod.make_noise((1, 1, 64, Y.shape[-1]), nd, seed=40 + i)):
+            smp, _ = m.get_pc_sampler("reverse_diffusion", "ald", Y, N=3, corrector_steps=1, snr=0.5)()
+        out[f"files_enh{i}"] = _np((m.to_audio(smp.squeeze(), n) * norm).squeeze())
+    skel["ncsnpp_48k"] = score_model_skeleton(refshim.make_score_model("ncsnpp_48k", seed=0, **REF_48K))
+    skel["ncsnpp_v2_sbve"] = score_model_skeleton(refshim.make_score_model("ncsnpp_v2", seed=0, **REF_V2_SBVE))
+    out["score_models"] = np.array(json.dumps(skel, separators=(",", ":")))
+    np.savez_compressed(os.path.join(OUT, f"{name}.npz"), **out)
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     golden_ops()
@@ -303,7 +430,13 @@ def main():
     golden_ode_v2()
     golden_mid_tc()
     golden_full_n30()            # ~2.5 minutes: the full-size reference run
+    golden_reference_live()
 
 
 if __name__ == "__main__":
-    main()
+    import sys
+    if sys.argv[1:] == ["reference_live"]:        # this fixture alone: leaves the others untouched
+        os.makedirs(OUT, exist_ok=True)
+        golden_reference_live()
+    else:
+        main()

@@ -6,16 +6,20 @@ with the same injected noise.  Second half: the in-training evaluation flow (mod
 ``install(rebind_forward="no_grad", refresh_on_eval=True)``, weights change, the EMA swap of ``eval()`` -- reached the way
 Lightning + DDP reach it, through ``nn.Module.eval(wrapper)`` -- and ``enhance`` must follow the swapped-in weights.
 
-Run on the B200 box: ``pytest -m gpu``.  Skipped when neither /root/reference nor oracle/_ref is present.
+Run on the B200 box: ``pytest -m gpu``.  The tests that install on a live ScoreModel are skipped when neither /root/reference
+nor oracle/_ref is present; the batched file service is compared with the reference's per-file loop as stored in
+tests/golden/reference_live.npz and runs from the repository alone.
 """
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import refshim, sde as o_sde, pipeline as o_pipe
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not refshim.reference_available(), reason="reference not staged (oracle/_ref) and no live checkout")]
+pytestmark = pytest.mark.gpu
+live = pytest.mark.skipif(not refshim.reference_available(), reason="reference not staged (oracle/_ref) and no live checkout")
 
 # mid-size config: 64..128 channels -> the tcgen05 convolutions run in fp16_tc mode (same as MID_E in test_gpu_parity.py)
 MID = dict(nf=64, ch_mult=(1, 2, 2), image_size=64, attn_resolutions=(16,), num_res_blocks=1, n_fft=126, hop_length=32)
@@ -50,6 +54,7 @@ def reference_run(model, wav, draws, n=N):
     return Y, sample, x_hat.squeeze().numpy(), nfe
 
 
+@live
 @pytest.mark.parametrize("mode", ["fp32", "fp16_tc"])
 def test_install_on_a_live_reference_score_model(mode):
     import sgmse_b200
@@ -125,6 +130,7 @@ class TinyEMA:
         pass
 
 
+@live
 def test_in_training_evaluation_follows_the_ema_swap():
     """validation_step (model.py:205-257) calls self.enhance per file with whatever weights eval() swapped into self.dnn;
     evaluate_model (util/inference.py:47-50) calls model.get_pc_sampler the same way.  The engine must see the EMA
@@ -185,21 +191,26 @@ def test_in_training_evaluation_follows_the_ema_swap():
         eng.close()
 
 
-def test_batched_file_service_against_the_reference_file_loop():
+def test_batched_file_service_against_the_reference_file_loop(golden_dir):
     """SURVEY.md §8f-2 against the REFERENCE (not against the engine itself): clips of three different lengths -- two padded
     frame counts, so two buckets -- through the unmodified reference's per-file loop (enhancement.py:58-99 on the CPU, injected
-    noise) and through BatchedEnhancer with the same per-clip noise; every clip individually, in both engine modes."""
-    import sgmse_b200
-    from sgmse_b200 import BatchedEnhancer, engine_from_score_model
-    model = make_model(seed=7)
+    noise; stored by oracle/make_golden.py: golden_reference_live, weights = oracle init seed 7) and through BatchedEnhancer
+    with the same weights and per-clip noise; every clip individually, in both engine modes."""
+    from oracle import weights as o_w
+    from oracle.arch import NetConfig
+    from sgmse_b200 import BatchedEnhancer, Engine, EngineConfig
+    gold = np.load(os.path.join(golden_dir, "reference_live.npz"))
+    net = {k: v for k, v in MID.items() if k not in ("n_fft", "hop_length")}
+    sd = o_w.make_state_dict(NetConfig.ncsnpp(**net), seed=7)
     g = torch.Generator().manual_seed(8)
     lengths = [4000, 1900, 3100, 2000]                      # 126, 60, 97, 63 frames -> padded to 128, 64, 128, 64
     clips = [0.1 * torch.randn(n, generator=g) * (1.0 + 0.5 * i) for i, n in enumerate(lengths)]
     nd = o_sde.n_noise_draws(N, "reverse_diffusion", "ald", 1)
     draws = {i: o_sde.make_noise((1, 1, 64, 128 if lengths[i] > 2048 else 64), nd, seed=40 + i) for i in range(len(clips))}
-    refs = [reference_run(model, c[None], draws[i])[2] for i, c in enumerate(clips)]
+    refs = [gold[f"files_enh{i}"] for i in range(len(clips))]
     for mode, tol in (("fp32", 1e-5), ("fp16_tc", 2.2e-3)):
-        eng = engine_from_score_model(model, mode=mode, max_batch=2)
+        eng = Engine(EngineConfig(**MID, mode=mode, max_batch=2))
+        eng.load_state_dict(sd)
         outs, ids = BatchedEnhancer(eng)(clips, seed=0, N=N, predictor="reverse_diffusion", corrector="ald", corrector_steps=1, snr=0.5,
                                          noise_for=lambda i, tp: torch.stack(draws[i]))
         errs = [rel_l2(o, r) for o, r in zip(outs, refs)]
